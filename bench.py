@@ -6,6 +6,7 @@ One "step" = one denoiser forward on one synthetic latent [1,4,64,32,32] with T5
 
     python bench.py --gpus N --steps K --warmup W          # our arm (N>1 under torchrun)
     python bench.py --impl reference ...                   # the reference's CPU arithmetic (oracle port)
+    python bench.py ... --dump-outputs DIR                 # also write the last timed step's output as DIR/*.npy
 
 JSON line keys follow the driver's contract: `value` is device-resident throughput, `e2e` is the same
 metric through the public model API with pinned-host inputs copied in and the result copied out
@@ -474,6 +475,20 @@ def mmdit_leg(timeout_s: float = 180.0):
         return {"error": repr(e)[:300]}
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """Writes each tensor as `out_dir/<name>.npy` in float32 (whole: the denoiser output of one step is 2 MB)."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    host = {k: v.detach().float().cpu().numpy() for k, v in arrays.items()}
+    assert sum(a.nbytes for a in host.values()) <= DUMP_LIMIT_BYTES
+    for k, a in host.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -495,7 +510,12 @@ def main():
     ap.add_argument("--profile-step", action="store_true",
                     help="after warm-up, bracket ONE step with cudaProfilerStart/Stop and exit (for `ncu --profile-from-start off`: "
                          "the launch list of exactly one step; prints no bench line)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed (the denoiser output, float32) as DIR/<name>.npy; the inputs "
+                         "and weights are seeded, so two builds run with the same arguments can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "osb200" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -597,6 +617,8 @@ def main():
         clocks.start()
     l0 = osb200.launch_count()
     ms = timed(step_resident, args.steps)
+    # a graph replay returns its static output buffer, which the e2e steps below overwrite: keep a copy of this one
+    last_out = out_holder["o"].clone() if args.dump_outputs else None
     launches = osb200.launch_count() - l0
     if replay is not None:   # a replay re-issues the captured kernels without passing through the C ABI counter
         launches = graph_launches * args.steps
@@ -642,6 +664,8 @@ def main():
         if world > 1:
             _finish(dist)
         return
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"stdit3_out": last_out})
     pk = peaks()
     g = fam.get("gemm", [0.0, 1.0, 1])
     gemm_tflops = g[0] / (g[1] * 1e-3) / 1e12
